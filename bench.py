@@ -18,6 +18,11 @@ barrier + synchronize on both sides of the timed region, max over ranks.  ``e2e`
 with the step's inputs copied from pinned host memory and the loss read back every step; the copy of step i+1 is
 prefetched on a side stream into a double buffer while step i computes (same loop for both arms,
 ``RFA_BENCH_E2E_PREFETCH=0`` serialises copy and compute again).
+
+``--dump-outputs DIR`` writes what the last timed step returned to its caller (the attention output and, for
+fwd_bwd, the gradients of the inputs) as float32 ``DIR/<name>.npy``, each cut down to the same fixed, seeded
+sample of token rows (``_rank<r>`` is appended to the name when N > 1).  Inputs are seeded too, so two builds run
+with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -49,7 +54,22 @@ def parse():
     ap.add_argument("--check", dest="check", action="store_true", default=True,
                     help="verify one untimed step against the fp32 oracle on sampled rows (default: on, ours only)")
     ap.add_argument("--no-check", dest="check", action="store_false")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's outputs as float32 DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_ROWS = 512  # token rows dumped over all ranks: 32 MiB of float32 at the headline shape
+
+
+def sample_rows(torch, arrays, world):
+    """The same seeded sample of token rows (dim 1) of every array, as float32 numpy arrays."""
+    n = next(iter(arrays.values())).shape[1]
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[: max(1, DUMP_ROWS // world)].sort().values
+    return {name: t.detach()[:, rows.to(t.device)].float().cpu().numpy() for name, t in arrays.items()}
 
 
 class ClockSampler:
@@ -276,10 +296,11 @@ def main():
         barrier()
         evs = []
         for _ in range(steps):
+            last.clear()  # the previous step's result is released before this step allocates its own
             flush.fill_(1)  # evict L2 between timed iterations (outside the events)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            run()
+            last.append(run())
             b.record()
             evs.append((a, b))
         barrier()
@@ -293,6 +314,7 @@ def main():
         return float(t[1])
 
     stats = {}
+    last = []  # what the last timed step returned
     launches = None
     if args.impl == "ours":
         from ring_flash_attn_b200.ops import cuda_ext
@@ -313,6 +335,14 @@ def main():
     step_stats = dict(stats)
     if args.impl == "ours":
         launches = counter.value
+    dumped = None
+    if args.dump_outputs:
+        arrays = {"out": last[0]}
+        if args.mode == "fwd_bwd":
+            arrays.update(zip(["dqkv"] if api == "qkvpacked" else ["dq", "dkv"], (t.grad for t in dev_in)))
+        dumped = sample_rows(torch, arrays, world)
+        del arrays
+    last.clear()
     e2e = None
     if not args.no_e2e:
         pipeline = "serial copy -> compute"
@@ -335,6 +365,12 @@ def main():
         e2e = {"value": 1000.0 / e2e_ms, "unit": "iter/s", "ms_per_step": e2e_ms,
                "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": 4, "input_pipeline": pipeline}
     clocks = sampler.stop() if rank == 0 else None
+    if dumped is not None:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ("" if world == 1 else f"_rank{rank}") + ".npy"), a)
 
     if rank == 0:
         value = 1000.0 / ms

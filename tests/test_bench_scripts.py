@@ -100,6 +100,32 @@ def test_prefetched_e2e_loop_pipelines_one_copy_per_step():
     assert ptrs[0] == ptrs[2] == ptrs[4] and ptrs[1] == ptrs[3] and ptrs[0] != ptrs[1]  # double buffer alternates
 
 
+def test_dump_sample_is_fixed_float32_and_small():
+    """bench.sample_rows (what ``--dump-outputs`` writes): the same token rows of every array on every run, exact
+    float32 copies of the bf16 values, and at most 64 MB at the headline shape whatever the GPU count."""
+    import importlib.util
+
+    import torch
+
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+
+    tokens = 2048
+    pos = torch.arange(tokens, dtype=torch.float32).view(1, tokens, 1, 1).expand(1, tokens, 2, 4).contiguous()
+    arrays = {"out": pos, "dqkv": torch.randn(1, tokens, 3, 2, 4, dtype=torch.bfloat16).requires_grad_(True)}
+    a, b = bench.sample_rows(torch, arrays, 1), bench.sample_rows(torch, arrays, 1)
+    rows = a["out"][0, :, 0, 0].astype(int)
+    assert a.keys() == arrays.keys() and all(x.dtype.name == "float32" for x in a.values())
+    assert a["out"].shape == (1, bench.DUMP_ROWS, 2, 4) and a["dqkv"].shape == (1, bench.DUMP_ROWS, 3, 2, 4)
+    assert all((a[k] == b[k]).all() for k in a)  # same rows every run
+    assert (rows[1:] > rows[:-1]).all()
+    assert (a["dqkv"] == arrays["dqkv"].detach()[:, rows].float().numpy()).all()  # same rows, exact values
+    assert bench.sample_rows(torch, arrays, 8)["out"].shape[1] == bench.DUMP_ROWS // 8
+    per_row = 32 * 128 * 4 * (1 + 3)  # out + dqkv of one headline token row, float32
+    assert bench.DUMP_ROWS * per_row <= 64 * 2**20
+
+
 def test_minimal_example_world2():
     """examples/ring_attention_minimal.py: shard, attend, backward, sampled fp32 check - on gloo."""
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr",
